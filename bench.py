@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus 8 --steps 5 --warmup 3
     python bench.py --impl reference ...      # unmodified NVIDIA/Megatron-LM from baseline/_ref
+    python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs OUT   # + OUT/*.npy: loss and weight sample after the last timed step
 
 Both arms print ONE JSON line on rank 0 with the IDENTICAL ``metric`` string and the same workload:
 
@@ -69,7 +70,15 @@ def parse():
     ap.add_argument("--vp", type=int, default=None)
     ap.add_argument("--ep", type=int, default=None)
     ap.add_argument("--dispatcher", default=None, help="MoE token dispatcher: alltoall | allgather | flex (NVLink push/pull)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="repo arm: after the timed steps, write what the last timed step computed (its loss, every timed step's loss and a fixed, seeded sample of "
+                         "the updated weights) to DIR/<name>.npy, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs is implemented for --impl b200")
+    return args
 
 
 # BASELINE.json configs 3-5: (tp, pp, vp, ep) for 8 GPUs, global batch, recompute, main-grad dtype, sequence parallel
@@ -197,14 +206,40 @@ def deterministic_init(torch, named_params, tp_rank, tp_world, num_layers):
     return n
 
 
+DUMP_SAMPLES_PER_PARAM = 4096      # 291 Llama-3-8B tensors -> 1.2 M fp32 values, 4.5 MiB: far below the 64 MiB the dump may take
+
+
+def dump_outputs(torch, out_dir, model_chunks, timed_losses):
+    """What the timed path computed in its last step, as float32 ``.npy`` files: ``loss.npy`` (that step's mean loss), ``loss_by_step.npy`` (one value
+    per timed step) and ``param_sample.npy`` — this rank's updated weights, for each parameter (in ``named_parameters`` order) the elements at
+    ``DUMP_SAMPLES_PER_PARAM`` flat indices drawn by a CPU generator seeded with crc32(name), so the same positions are sampled in every run."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    losses = torch.stack([l.detach().float().reshape(()) for l in timed_losses]).cpu().numpy()
+    samples = []
+    with torch.no_grad():
+        for chunk in model_chunks:
+            for name, p in chunk.named_parameters():
+                name = name.replace("module.", "")
+                flat = p.detach().reshape(-1)
+                g = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+                idx = torch.randint(0, flat.numel(), (min(flat.numel(), DUMP_SAMPLES_PER_PARAM),), generator=g)
+                samples.append(flat[idx.to(flat.device)].float().cpu())
+    np.save(os.path.join(out_dir, "loss.npy"), losses[-1:].astype(np.float32))
+    np.save(os.path.join(out_dir, "loss_by_step.npy"), losses.astype(np.float32))
+    np.save(os.path.join(out_dir, "param_sample.npy"), torch.cat(samples).numpy().astype(np.float32))
+
+
 def losses_to_dict(torch, loss_tensors):
     vals = torch.stack([l.detach().float().reshape(()) for l in loss_tensors]).cpu().tolist() if loss_tensors else []
     return {str(i + 1): round(float(v), 5) for i, v in enumerate(vals)}
 
 
 # ------------------------------------------------------------------------------------------------
-def _b200_variant(args, torch, dist, rank, world, local, *, sequence_parallel, recompute, main_grads_fp32, want_e2e, sample_clocks):
-    """Build a TrainEngine, run W warm-up + K timed steps (+ the e2e loop).  Returns a dict of plain floats."""
+def _b200_variant(args, torch, dist, rank, world, local, *, sequence_parallel, recompute, main_grads_fp32, want_e2e, sample_clocks, dump_dir=None):
+    """Build a TrainEngine, run W warm-up + K timed steps (+ the e2e loop).  Returns a dict of plain floats.  With ``dump_dir``, rank 0 writes the
+    outputs of the last timed step there before the e2e loop changes the weights."""
     from megatron_b200 import ops
     from megatron_b200.training.engine import TrainEngine
 
@@ -243,6 +278,8 @@ def _b200_variant(args, torch, dist, rank, world, local, *, sequence_parallel, r
     ms, _wall = timed_loop(torch, dist, step_dev, args.steps, world)
     launches = ops.launch_count()
     clocks = sampler.stop() if (rank == 0 and sample_clocks) else {}
+    if dump_dir and rank == 0:
+        dump_outputs(torch, dump_dir, eng.model_chunks, losses[args.warmup:])
     tokens_per_step = args.global_batch * eng.seq_length
     res = {"value": tokens_per_step * args.steps / (ms / 1e3), "ms_per_step": ms / args.steps, "gpu_launches": launches, "clocks": clocks,
            "tflops_per_gpu": eng.flops_per_step * args.steps / (ms / 1e3) / world / 1e12, "seq_length": eng.seq_length, "params_initialised": n_init}
@@ -318,6 +355,12 @@ def run_b200_other(args):
     ms, _ = timed_loop(torch, dist, step_dev, args.steps, world)
     launches = ops.launch_count()
     clocks = sampler.stop() if rank == 0 else {}
+    if args.dump_outputs:
+        # the loss lives on the last pipeline stage: rank 0 writes the max over ranks of each timed step's value (other stages report 0)
+        timed = torch.stack([l.detach().float().reshape(()) for l in losses[args.warmup:]]).cuda()
+        dist.all_reduce(timed, op=dist.ReduceOp.MAX)
+        if rank == 0:
+            dump_outputs(torch, args.dump_outputs, eng.model_chunks, list(timed))
     tokens_per_step = gb * eng.seq_length
     value = tokens_per_step * args.steps / (ms / 1e3)
     e2e = None
@@ -378,7 +421,7 @@ def run_b200(args):
         recompute = dict(recompute_granularity="selective", recompute_modules=args.recompute.split(","))
 
     main = _b200_variant(args, torch, dist, rank, world, local, sequence_parallel=False, recompute=recompute, main_grads_fp32=fp32_grads,
-                         want_e2e=not args.no_e2e, sample_clocks=True)
+                         want_e2e=not args.no_e2e, sample_clocks=True, dump_dir=args.dump_outputs)
     # fused-vs-NCCL self check of every GEMM<->collective pair op on this model's shapes (N >= 2)
     pair_err = None
     if world > 1:
@@ -449,7 +492,7 @@ def run_reference(args):
     selective(core_attn) recompute, fp32 main grads, identical initial weights and tokens."""
     ref = os.path.join(REPO, "baseline", "_ref")
     if not os.path.isdir(os.path.join(ref, "megatron", "core")):
-        print(json.dumps({"impl": "reference", "unavailable": "baseline/_ref is not installed (pip install --no-deps --target baseline/_ref /root/reference)"}))
+        print(json.dumps({"impl": "reference", "unavailable": "baseline/_ref is not installed (pip install --no-deps --target baseline/_ref <Megatron-LM checkout>)"}))
         return
     sys.path.insert(0, ref)
     sys.path = [p for p in sys.path if os.path.abspath(p or ".") != REPO]

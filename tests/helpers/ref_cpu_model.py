@@ -104,6 +104,7 @@ def init_params(named_params, tp_rank, tp_world):
 
 
 CFG = dict(num_layers=2, hidden_size=64, ffn_hidden_size=128, num_attention_heads=4, num_query_groups=2, kv_channels=16, vocab=128, seq=32, batch=2)
+CFG.update(json.loads(os.environ.get("REF_MODEL_SIZE", "{}")))          # the checkpoint-interop runs use a smaller model
 
 
 # REF_VARIANT=moe: 4 experts, top-2, softmax-then-top-k router with the switch aux loss, all-gather dispatcher, one expert MLP per expert (no grouped GEMM)

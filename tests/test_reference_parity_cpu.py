@@ -1,39 +1,43 @@
-"""Loss and gradient parity with the UNMODIFIED reference (``baseline/_ref``, megatron-core 0.20.0) on identical weights and tokens.
+"""Loss and gradient parity with the UNMODIFIED reference (megatron-core 0.20.0) on identical weights and tokens.
 
 The same name-seeded full-tensor initialisation that ``bench.py`` applies to both arms is applied to a tiny Llama-style GPT in both
 frameworks (TP=1 and TP=2 over gloo); forward loss and every parameter gradient must agree to fp32 round-off.  This is the contract
 behind ``bench.py``'s ``loss_by_step`` comparison: same parameter names, same shard layout (interleaved QKV groups, [gate; up] fc1
-halves), same math.  Skipped when the reference is not installed."""
+halves), same math.
+
+What the reference computed is stored under ``tests/golden/reference/`` (``tests/helpers/make_reference_golden.py`` regenerates it from an
+install of the reference): losses, learning rates and norms in full; per tensor its shape, max |x|, sum, L2 norm and the values at a fixed
+sample of elements; the reference's own checkpoints of the interop model; dataset samples; schedule tables."""
+import json
 import os
-import subprocess
 import sys
 
 import pytest
 import torch
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(REPO, "baseline", "_ref", "megatron", "core")
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="baseline/_ref (the reference install) is absent")
+GOLDEN = os.path.join(REPO, "tests", "golden", "reference")
 
 
-def _run_reference(tmp_path, tp, variant="", world=None):
-    import socket
+def _reference(name):
+    """Per-rank results of the reference run ``name``."""
+    with open(os.path.join(GOLDEN, f"model_{name}.json")) as f:
+        return json.load(f)
 
-    world = world or tp
 
-    with socket.socket() as s:
-        s.bind(("127.0.0.1", 0))
-        port = s.getsockname()[1]
-    prefix = str(tmp_path / f"ref_tp{tp}")
-    procs = []
-    for r in range(world):
-        env = dict(os.environ, RANK=str(r), WORLD_SIZE=str(world), MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), OMP_NUM_THREADS="1", REF_VARIANT=variant)
-        procs.append(subprocess.Popen([sys.executable, os.path.join(REPO, "tests", "helpers", "ref_cpu_model.py"), prefix, str(tp)], env=env,
-                                      stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True))
-    for p in procs:
-        out, _ = p.communicate(timeout=600)
-        assert p.returncode == 0, out[-3000:]
-    return [torch.load(f"{prefix}.rank{r}.pt") for r in range(world)]
+def _assert_tensors_match(got, want, tol, what, relative=True):
+    """Every tensor of ``want`` against this framework's full tensor in ``got``.  Each check follows from max |got - ref| < tol * scale, with
+    scale = max |ref| (``relative``) or 1."""
+    for n, w in want.items():
+        g = got[n].detach().double()
+        assert list(g.shape) == w["shape"], (what, n, list(g.shape), w["shape"])
+        scale = max(w["absmax"], 1e-12) if relative else 1.0
+        bound = tol * scale
+        err = float((g.flatten()[w["idx"]] - torch.tensor(w["val"], dtype=torch.float64)).abs().max()) / scale
+        assert err < tol, f"{what} {n}: err {err}"
+        assert abs(float(g.abs().max()) - w["absmax"]) < bound, f"{what} {n}: max |x| {float(g.abs().max())} vs {w['absmax']}"
+        assert abs(float(g.sum()) - w["sum"]) < bound * g.numel(), f"{what} {n}: sum {float(g.sum())} vs {w['sum']}"
+        assert abs(float(g.norm()) - w["norm"]) < bound * g.numel() ** 0.5, f"{what} {n}: norm {float(g.norm())} vs {w['norm']}"
 
 
 def _ours(rank, world, tp, variant=""):
@@ -99,29 +103,24 @@ def _ours(rank, world, tp, variant=""):
 def test_loss_and_grad_parity_with_reference(tmp_path, tp):
     from dist_utils import run_distributed
 
-    ref = _run_reference(tmp_path, tp)
+    ref = _reference(f"gpt_tp{tp}")
     ours = run_distributed(_ours, tp, tp)
     for r in range(tp):
         assert sorted(ours[r]["names"]) == sorted(ref[r]["grads"].keys()), "parameter names differ from the reference's"
         assert abs(ours[r]["loss"] - ref[r]["loss"]) < 2e-5, (ours[r]["loss"], ref[r]["loss"])
-        for n, g in ref[r]["grads"].items():
-            go = ours[r]["grads"][n]
-            err = float((go - g).abs().max() / g.abs().max().clamp(min=1e-12))
-            assert err < 2e-4, f"rank {r} grad {n}: rel err {err}"
+        _assert_tensors_match(ours[r]["grads"], ref[r]["grads"], 2e-4, f"rank {r} grad")
 
 
 def test_moe_loss_and_grad_parity_with_reference(tmp_path):
     """A 4-expert top-2 MoE GPT (router + aux loss, all-gather dispatcher, per-expert MLPs): same parameter names, loss and gradients as the unmodified reference."""
     from dist_utils import run_distributed
 
-    ref = _run_reference(tmp_path, 1, "moe")[0]
+    ref = _reference("moe")[0]
     ours = run_distributed(_ours, 1, 1, "moe")[0]
     assert sorted(ours["names"]) == sorted(ref["grads"].keys()), (sorted(set(ours["names"]) ^ set(ref["grads"].keys())))
     assert any("router" in n for n in ours["names"]) and any("local_experts" in n for n in ours["names"])
     assert abs(ours["loss"] - ref["loss"]) < 2e-5, (ours["loss"], ref["loss"])
-    for n, g in ref["grads"].items():
-        err = float((ours["grads"][n] - g).abs().max() / g.abs().max().clamp(min=1e-12))
-        assert err < 5e-4, f"grad {n}: rel err {err}"
+    _assert_tensors_match(ours["grads"], ref["grads"], 5e-4, "grad")
 
 
 def test_moe_deepseek_style_router_parity_with_reference(tmp_path):
@@ -129,14 +128,12 @@ def test_moe_deepseek_style_router_parity_with_reference(tmp_path):
     unmodified reference's."""
     from dist_utils import run_distributed
 
-    ref = _run_reference(tmp_path, 1, "moe_dsv3")[0]
+    ref = _reference("moe_dsv3")[0]
     ours = run_distributed(_ours, 1, 1, "moe_dsv3")[0]
     assert sorted(ours["names"]) == sorted(ref["grads"].keys()), sorted(set(ours["names"]) ^ set(ref["grads"].keys()))
     assert any("shared_experts" in n for n in ours["names"])
     assert abs(ours["loss"] - ref["loss"]) < 2e-5, (ours["loss"], ref["loss"])
-    for n, g in ref["grads"].items():
-        err = float((ours["grads"][n] - g).abs().max() / g.abs().max().clamp(min=1e-12))
-        assert err < 1e-3, f"grad {n}: rel err {err}"
+    _assert_tensors_match(ours["grads"], ref["grads"], 1e-3, "grad")
 
 
 def test_moe_capacity_drop_and_pad_parity_with_reference(tmp_path):
@@ -144,13 +141,11 @@ def test_moe_capacity_drop_and_pad_parity_with_reference(tmp_path):
     gradient equal the unmodified reference's."""
     from dist_utils import run_distributed
 
-    ref = _run_reference(tmp_path, 1, "moe_drop")[0]
+    ref = _reference("moe_drop")[0]
     ours = run_distributed(_ours, 1, 1, "moe_drop")[0]
     assert sorted(ours["names"]) == sorted(ref["grads"].keys())
     assert abs(ours["loss"] - ref["loss"]) < 2e-5, (ours["loss"], ref["loss"])
-    for n, g in ref["grads"].items():
-        err = float((ours["grads"][n] - g).abs().max() / g.abs().max().clamp(min=1e-12))
-        assert err < 1e-3, f"grad {n}: rel err {err}"
+    _assert_tensors_match(ours["grads"], ref["grads"], 1e-3, "grad")
 
 
 def test_mup_parity_with_reference(tmp_path, monkeypatch):
@@ -160,13 +155,11 @@ def test_mup_parity_with_reference(tmp_path, monkeypatch):
 
     plain = run_distributed(_ours, 1, 1, "")[0]
     monkeypatch.setenv("REF_CFG_OVERRIDE", '{"use_mup": true, "mup_base_hidden_size": 32, "mup_embedding_mult": 2.0}')
-    ref = _run_reference(tmp_path, 1, "")[0]
+    ref = _reference("mup")[0]
     ours = run_distributed(_ours, 1, 1, "")[0]
     assert abs(ours["loss"] - plain["loss"]) > 1e-3
     assert abs(ours["loss"] - ref["loss"]) < 2e-5, (ours["loss"], ref["loss"])
-    for n, g in ref["grads"].items():
-        err = float((ours["grads"][n] - g).abs().max() / g.abs().max().clamp(min=1e-12))
-        assert err < 1e-3, f"grad {n}: rel err {err}"
+    _assert_tensors_match(ours["grads"], ref["grads"], 1e-3, "grad")
 
 
 def test_moe_expert_parallel_parity_with_reference(tmp_path):
@@ -175,14 +168,12 @@ def test_moe_expert_parallel_parity_with_reference(tmp_path):
     equal the unmodified reference's."""
     from dist_utils import run_distributed
 
-    ref = _run_reference(tmp_path, 1, "moe_ep2", world=2)
+    ref = _reference("moe_ep2")
     ours = run_distributed(_ours, 2, 1, "moe_ep2")
     for r in range(2):
         assert sorted(ours[r]["names"]) == sorted(ref[r]["grads"].keys())
         assert abs(ours[r]["loss"] - ref[r]["loss"]) < 2e-5, (r, ours[r]["loss"], ref[r]["loss"])
-        for n, g in ref[r]["grads"].items():
-            err = float((ours[r]["grads"][n] - g).abs().max() / g.abs().max().clamp(min=1e-12))
-            assert err < 5e-4, f"rank {r} grad {n}: rel err {err}"
+        _assert_tensors_match(ours[r]["grads"], ref[r]["grads"], 5e-4, f"rank {r} grad")
 
 
 def _ours_bert(rank, world):
@@ -223,13 +214,11 @@ def test_bert_parity_with_reference(tmp_path):
     """BERT (token types, learned positions, padding mask, LM head, pooler + binary head): parameter names, loss and gradients equal the unmodified reference's."""
     from dist_utils import run_distributed
 
-    ref = _run_reference(tmp_path, 1, "bert")[0]
+    ref = _reference("bert")[0]
     ours = run_distributed(_ours_bert, 1)[0]
     assert sorted(ours["names"]) == sorted(ref["grads"].keys()), sorted(set(ours["names"]) ^ set(ref["grads"].keys()))
     assert abs(ours["loss"] - ref["loss"]) < 2e-5, (ours["loss"], ref["loss"])
-    for n, g in ref["grads"].items():
-        err = float((ours["grads"][n] - g).abs().max() / g.abs().max().clamp(min=1e-12))
-        assert err < 5e-4, f"grad {n}: rel err {err}"
+    _assert_tensors_match(ours["grads"], ref["grads"], 5e-4, "grad")
 
 
 def _ours_t5(rank, world):
@@ -281,13 +270,11 @@ def test_t5_parity_with_reference(tmp_path):
     """T5 encoder-decoder (cross attention, padding / causal / cross masks, shared embeddings + LM-head bias): names, loss and gradients equal the reference's."""
     from dist_utils import run_distributed
 
-    ref = _run_reference(tmp_path, 1, "t5")[0]
+    ref = _reference("t5")[0]
     ours = run_distributed(_ours_t5, 1)[0]
     assert sorted(ours["names"]) == sorted(ref["grads"].keys()), sorted(set(ours["names"]) ^ set(ref["grads"].keys()))
     assert abs(ours["loss"] - ref["loss"]) < 2e-5, (ours["loss"], ref["loss"])
-    for n, g in ref["grads"].items():
-        err = float((ours["grads"][n] - g).abs().max() / g.abs().max().clamp(min=1e-12))
-        assert err < 5e-4, f"grad {n}: rel err {err}"
+    _assert_tensors_match(ours["grads"], ref["grads"], 5e-4, "grad")
 
 
 def _ours_vit(rank, world):
@@ -326,14 +313,12 @@ def test_clip_vit_parity_with_reference(tmp_path):
     """CLIP ViT tower (conv patch embedding, class token, learned positions, pre-norm): output shape, parameter names, loss and gradients equal the reference's."""
     from dist_utils import run_distributed
 
-    ref = _run_reference(tmp_path, 1, "vit")[0]
+    ref = _reference("vit")[0]
     ours = run_distributed(_ours_vit, 1)[0]
-    assert ours["shape"] == ref["shape"]
+    assert list(ours["shape"]) == ref["shape"]
     assert sorted(ours["names"]) == sorted(ref["grads"].keys()), sorted(set(ours["names"]) ^ set(ref["grads"].keys()))
     assert abs(ours["loss"] - ref["loss"]) < 1e-6, (ours["loss"], ref["loss"])
-    for n, g in ref["grads"].items():
-        err = float((ours["grads"][n] - g).abs().max() / g.abs().max().clamp(min=1e-12))
-        assert err < 5e-4, f"grad {n}: rel err {err}"
+    _assert_tensors_match(ours["grads"], ref["grads"], 5e-4, "grad")
 
 
 def _ours_optim(rank, world, dist_opt=False):
@@ -374,15 +359,13 @@ def test_optimizer_stack_parity_with_reference(tmp_path):
     warm-up from 0 then cosine decay): losses, gradient norms, learning rates and the final parameters equal the unmodified reference's."""
     from dist_utils import run_distributed
 
-    ref = _run_reference(tmp_path, 1, "optim")[0]
+    ref = _reference("optim")[0]
     ours = run_distributed(_ours_optim, 1)[0]
     assert all(abs(a - b) < 2e-5 for a, b in zip(ours["losses"], ref["losses"])), (ours["losses"], ref["losses"])
     assert all(abs(a - b) < 1e-4 * b for a, b in zip(ours["grad_norms"], ref["grad_norms"])), (ours["grad_norms"], ref["grad_norms"])
     assert sorted(round(x, 9) for x in ours["lr"]) == sorted(round(x, 9) for x in ref["lr"]), (ours["lr"], ref["lr"])
     assert ours["losses"][2] < ours["losses"][0]
-    for n, p in ref["params"].items():
-        err = float((ours["params"][n] - p).abs().max())
-        assert err < 2e-5, f"param {n}: abs err {err} after 3 steps"
+    _assert_tensors_match(ours["params"], ref["params"], 2e-5, "param after 3 steps", relative=False)
 
 
 def test_distributed_optimizer_parity_with_reference(tmp_path):
@@ -390,14 +373,12 @@ def test_distributed_optimizer_parity_with_reference(tmp_path):
     the global gradient norm and every rank's parameters after three steps equal the unmodified reference's."""
     from dist_utils import run_distributed
 
-    ref = _run_reference(tmp_path, 1, "distopt", world=2)
+    ref = _reference("distopt")
     ours = run_distributed(_ours_optim, 2, True)
     for r in range(2):
         assert all(abs(a - b) < 2e-5 for a, b in zip(ours[r]["losses"], ref[r]["losses"])), (r, ours[r]["losses"], ref[r]["losses"])
         assert all(abs(a - b) < 1e-4 * b for a, b in zip(ours[r]["grad_norms"], ref[r]["grad_norms"])), (ours[r]["grad_norms"], ref[r]["grad_norms"])
-        for n, p in ref[r]["params"].items():
-            err = float((ours[r]["params"][n] - p).abs().max())
-            assert err < 2e-5, f"rank {r} param {n}: abs err {err} after 3 steps"
+        _assert_tensors_match(ours[r]["params"], ref[r]["params"], 2e-5, f"rank {r} param after 3 steps", relative=False)
     assert all(torch.equal(ours[0]["params"][n], ours[1]["params"][n]) for n in ours[0]["params"])        # replicas stay in sync
 
 
@@ -452,39 +433,44 @@ def test_pipeline_schedule_parity_with_reference(tmp_path):
     unmodified reference's schedule (same loss scaling by the number of micro-batches, same p2p tensor flow)."""
     from dist_utils import run_distributed
 
-    ref = _run_reference(tmp_path, 1, "pp2", world=2)
+    ref = _reference("pp2")
     ours = run_distributed(_ours_pp2, 2)
     assert ours[0]["losses"] == [] and len(ours[1]["losses"]) == 4
     assert all(abs(a - b) < 2e-5 for a, b in zip(ours[1]["losses"], ref[1]["losses"])), (ours[1]["losses"], ref[1]["losses"])
     for r in range(2):
         assert sorted(ours[r]["grads"]) == sorted(ref[r]["grads"]), (r, sorted(set(ours[r]["grads"]) ^ set(ref[r]["grads"])))
-        for n, g in ref[r]["grads"].items():
-            err = float((ours[r]["grads"][n] - g).abs().max() / g.abs().max().clamp(min=1e-12))
-            assert err < 5e-4, f"stage {r} grad {n}: rel err {err}"
+        _assert_tensors_match(ours[r]["grads"], ref[r]["grads"], 5e-4, f"stage {r} grad")
 
 
 # ---- distributed-checkpoint interop (SURVEY 7.4-6: "cross-load a checkpoint with the reference") --------------------------------------
 
 
-def _spawn_reference(tmp_path, tp, *extra):
-    import socket
-
-    with socket.socket() as s:
-        s.bind(("127.0.0.1", 0))
-        port = s.getsockname()[1]
-    prefix = str(tmp_path / f"ref_{extra[0]}_tp{tp}")
-    procs = []
-    for r in range(tp):
-        env = dict(os.environ, RANK=str(r), WORLD_SIZE=str(tp), MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), OMP_NUM_THREADS="1")
-        procs.append(subprocess.Popen([sys.executable, os.path.join(REPO, "tests", "helpers", "ref_cpu_model.py"), prefix, str(tp), *extra], env=env,
-                                      stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True))
-    for p in procs:
-        out, _ = p.communicate(timeout=600)
-        assert p.returncode == 0, out[-3000:]
-    return prefix
+# The interop model is smaller than the parity model so that the reference's checkpoints of it can be stored (keys of ``CFG`` in ref_cpu_model.py).
+CKPT_MODEL = dict(hidden_size=16, ffn_hidden_size=32, kv_channels=4, vocab=32, seq=8)
 
 
-def _our_model(tp):
+def _reference_checkpoint(tmp_path, tp):
+    """Unpack the reference's checkpoint written at TP=tp."""
+    import tarfile
+
+    dst = tmp_path / f"ckpt_ref_tp{tp}"
+    with tarfile.open(os.path.join(GOLDEN, f"ckpt_tp{tp}.tar.gz")) as tar:
+        tar.extractall(dst, filter="data")
+    return dst
+
+
+def _dcp_tensors(ckpt_dir):
+    """Every tensor of a torch_dist checkpoint, read in full by torch.distributed.checkpoint (the reader both frameworks load through)."""
+    import torch.distributed.checkpoint as dcp
+    from torch.distributed.checkpoint.metadata import TensorStorageMetadata
+
+    md = dcp.FileSystemReader(str(ckpt_dir)).read_metadata()
+    sd = {k: torch.empty(list(m.size), dtype=m.properties.dtype) for k, m in md.state_dict_metadata.items() if isinstance(m, TensorStorageMetadata)}
+    dcp.load(sd, storage_reader=dcp.FileSystemReader(str(ckpt_dir)), no_dist=True)
+    return sd
+
+
+def _our_model(tp, num_layers=2, hidden_size=64, ffn_hidden_size=128, num_attention_heads=4, num_query_groups=2, kv_channels=16, vocab=128, seq=32):
     import torch.nn.functional as F
 
     from megatron_b200.core import parallel_state as ps
@@ -493,10 +479,11 @@ def _our_model(tp):
     from megatron_b200.core.transformer.transformer_config import TransformerConfig
 
     ps.initialize_model_parallel(tensor_model_parallel_size=tp)
-    cfg = TransformerConfig(num_layers=2, hidden_size=64, ffn_hidden_size=128, num_attention_heads=4, num_query_groups=2, kv_channels=16, normalization="RMSNorm",
+    cfg = TransformerConfig(num_layers=num_layers, hidden_size=hidden_size, ffn_hidden_size=ffn_hidden_size, num_attention_heads=num_attention_heads,
+                            num_query_groups=num_query_groups, kv_channels=kv_channels, normalization="RMSNorm",
                             gated_linear_unit=True, activation_func=F.silu, add_bias_linear=False, hidden_dropout=0.0, attention_dropout=0.0, use_cpu_initialization=True,
                             gradient_accumulation_fusion=False, perform_initialization=False, tensor_model_parallel_size=tp)
-    m = GPTModel(cfg, get_gpt_layer_local_spec(normalization="RMSNorm"), vocab_size=128, max_sequence_length=32, parallel_output=True,
+    m = GPTModel(cfg, get_gpt_layer_local_spec(normalization="RMSNorm"), vocab_size=vocab, max_sequence_length=seq, parallel_output=True,
                  share_embeddings_and_output_weights=False, position_embedding_type="rope", rotary_base=10000)
     return m, ps.get_tensor_model_parallel_rank()
 
@@ -526,7 +513,7 @@ def _seeded_init(m, tp_rank, tp):
 def _ours_save(rank, world, tp, ckpt_dir):
     from megatron_b200.core import dist_checkpointing
 
-    m, tp_rank = _our_model(tp)
+    m, tp_rank = _our_model(tp, **CKPT_MODEL)
     _seeded_init(m, tp_rank, tp)
     dist_checkpointing.save(m.sharded_state_dict(), ckpt_dir)
     return True
@@ -535,7 +522,7 @@ def _ours_save(rank, world, tp, ckpt_dir):
 def _ours_load(rank, world, tp, ckpt_dir):
     from megatron_b200.core import dist_checkpointing
 
-    m, tp_rank = _our_model(tp)
+    m, tp_rank = _our_model(tp, **CKPT_MODEL)
     with torch.no_grad():
         for _, p in m.named_parameters():
             p.zero_()
@@ -548,31 +535,33 @@ def _ours_load(rank, world, tp, ckpt_dir):
 
 @pytest.mark.parametrize("tp_write,tp_read", [(2, 1), (1, 2)])
 def test_reference_loads_our_checkpoint(tmp_path, tp_write, tp_read):
-    """A torch_dist checkpoint written by this framework (TP=tp_write) is read by the UNMODIFIED reference at another TP size."""
+    """A torch_dist checkpoint written by this framework (TP=tp_write) holds, under every key and global shape of the UNMODIFIED reference's own checkpoint
+    of the same model at TP=tp_read, exactly the tensors the reference wrote there: what the reference reads back at that TP size."""
     from dist_utils import run_distributed
 
     ckpt = tmp_path / "ckpt_ours"
     ckpt.mkdir()
     run_distributed(_ours_save, tp_write, tp_write, str(ckpt))
-    prefix = _spawn_reference(tmp_path, tp_read, "load", str(ckpt))
-    for r in range(tp_read):
-        res = torch.load(f"{prefix}.rank{r}.pt")
-        assert res["n_params"] == 15 and res["max_abs_diff"] == 0.0, res
+    ours, ref = _dcp_tensors(ckpt), _dcp_tensors(_reference_checkpoint(tmp_path, tp_read))
+    assert sorted(ours) == sorted(ref) and len(ref) > 0, sorted(set(ours) ^ set(ref))
+    for k, t in ref.items():
+        assert ours[k].dtype == t.dtype and torch.equal(ours[k], t), k
 
 
 @pytest.mark.parametrize("tp_write,tp_read", [(2, 1), (1, 2)])
 def test_we_load_reference_checkpoint(tmp_path, tp_write, tp_read):
-    """...and a checkpoint written by the reference is read by this framework, resharded."""
+    """...and a checkpoint written by the reference (stored) is read by this framework, resharded."""
     from dist_utils import run_distributed
 
-    ckpt = tmp_path / "ckpt_ref"
-    ckpt.mkdir()
-    _spawn_reference(tmp_path, tp_write, "save", str(ckpt))
+    ckpt = _reference_checkpoint(tmp_path, tp_write)
     diffs = run_distributed(_ours_load, tp_read, tp_read, str(ckpt))
     assert all(d == 0.0 for d in diffs), diffs
 
 
 # ---- data pipeline -----------------------------------------------------------------------------------------------------------------------------
+
+
+DATA_SEQ, DATA_SEED, DATA_SPLIT, DATA_COUNTS = 32, 1234, "80,15,5", [64, 12, 8]
 
 
 def _write_corpus(prefix, n_docs, seed):
@@ -588,52 +577,52 @@ def _write_corpus(prefix, n_docs, seed):
     b.finalize(prefix + ".idx")
 
 
+def write_corpora(d):
+    _write_corpus(os.path.join(d, "a"), 300, 1)
+    _write_corpus(os.path.join(d, "b"), 200, 2)
+
+
+def data_blend_args(d, blend):
+    return ["0.7", os.path.join(d, "a"), "0.3", os.path.join(d, "b")] if blend else ["1.0", os.path.join(d, "a")]
+
+
 @pytest.mark.parametrize("blend", [False, True])
 def test_gpt_dataset_samples_match_reference(tmp_path, blend):
-    """The reference reads the .bin/.idx files THIS framework writes, and both build the same train / valid / test samples from them (document shuffle, sample
+    """The reference read the .bin/.idx files THIS framework writes, and both build the same train / valid / test samples from them (document shuffle, sample
     index, blending of two corpora, loss masks, reset position ids) for the same seed — a run switched over sees the same data order."""
     from megatron_b200.core.datasets import BlendedMegatronDatasetBuilder, GPTDatasetConfig
     from megatron_b200.core.datasets.gpt_dataset import GPTDataset
     from megatron_b200.core.datasets.utils import get_blend_from_list
 
-    _write_corpus(str(tmp_path / "a"), 300, 1)
-    _write_corpus(str(tmp_path / "b"), 200, 2)
-    blend_args = ["0.7", str(tmp_path / "a"), "0.3", str(tmp_path / "b")] if blend else ["1.0", str(tmp_path / "a")]
-    counts = [64, 12, 8]
-    out = tmp_path / "ref.pt"
-    env = dict(os.environ, OMP_NUM_THREADS="1")
-    r = subprocess.run([sys.executable, os.path.join(REPO, "tests", "helpers", "ref_data.py"), str(out), str(tmp_path / "ref_cache"), "32", "1234", "80,15,5", *map(str, counts), *blend_args],
-                       env=env, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-3000:]
-    ref = torch.load(out)
+    write_corpora(str(tmp_path))
+    blend_args = data_blend_args(str(tmp_path), blend)
+    with open(os.path.join(GOLDEN, f"gpt_dataset_{'blend' if blend else 'single'}.json")) as f:
+        ref = json.load(f)
 
     class Tok:
         eod = 99
         unique_identifiers = {"class": "TestTokenizer", "eod": 99}
 
-    cfg = GPTDatasetConfig(random_seed=1234, sequence_length=32, blend=get_blend_from_list(blend_args), split="80,15,5", path_to_cache=str(tmp_path / "our_cache"), tokenizer=Tok(),
-                           reset_position_ids=True, reset_attention_mask=False, eod_mask_loss=True, create_attention_mask=False, mmap_bin_files=False)
-    ours = BlendedMegatronDatasetBuilder(GPTDataset, counts, lambda: True, cfg).build()
+    cfg = GPTDatasetConfig(random_seed=DATA_SEED, sequence_length=DATA_SEQ, blend=get_blend_from_list(blend_args), split=DATA_SPLIT, path_to_cache=str(tmp_path / "our_cache"),
+                           tokenizer=Tok(), reset_position_ids=True, reset_attention_mask=False, eod_mask_loss=True, create_attention_mask=False, mmap_bin_files=False)
+    ours = BlendedMegatronDatasetBuilder(GPTDataset, DATA_COUNTS, lambda: True, cfg).build()
     for name, ds in zip(("train", "valid", "test"), ours):
         assert (ds is None) == (ref[name] is None)
         if ds is None:
             continue
         assert len(ds) == ref[name]["len"], (name, len(ds), ref[name]["len"])
         for i, want in ref[name]["samples"].items():
-            got = ds[i]
-            for k, v in want.items():
+            got = ds[int(i)]
+            for k, (dtype, values) in want.items():
+                v = torch.tensor(values, dtype=getattr(torch, dtype))
                 assert torch.equal(torch.as_tensor(got[k]).to(v.dtype), v), (name, i, k)
 
 
 # ---- pure-Python subsystems: schedules, micro-batch ramp-up, rank enumeration ------------------------------------------------------------
 @pytest.fixture(scope="module")
 def ref_pure():
-    r = subprocess.run([sys.executable, os.path.join(REPO, "tests", "helpers", "ref_pure.py")], cwd="/tmp", capture_output=True, text=True, timeout=600)
-    line = [ln for ln in r.stdout.splitlines() if ln.startswith("JSON:")]
-    assert line, r.stdout[-2000:] + r.stderr[-2000:]
-    import json
-
-    return json.loads(line[0][5:])
+    with open(os.path.join(GOLDEN, "schedules_and_ranks.json")) as f:
+        return json.load(f)
 
 
 def _pure_cfg():

@@ -395,59 +395,41 @@ def test_telemetry_spans_and_metrics(tmp_path):
     assert m.values["train.tokens_per_second"] == 2000 and m.values["train.tflops_per_gpu"] == 2.0 and m.values["train.lm_loss"] == 3.0
 
 
-def _reference_flops_fn():
-    """The reference's analytic model, extracted from its source (pure python) — None when /root/reference is not there."""
-    import ast
-    import os
+def _reference_golden(name):
+    """Values computed by the unmodified reference (``tests/helpers/make_reference_golden.py``)."""
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference", name)) as f:
+        return json.load(f)
 
-    path = "/root/reference/megatron/training/training.py"
-    if not os.path.exists(path):
-        return None
-    src = open(path).read()
-    fn = [n for n in ast.parse(src).body if isinstance(n, ast.FunctionDef) and n.name == "num_floating_point_operations"][0]
-    ns = {}
-    exec("def is_linear_attention_variant(v): return v in ('gdn', 'gdn2', 'gated_delta_net')\n"
-         "def is_gated_delta_net_variant(v): return v in ('gdn', 'gdn2', 'gated_delta_net')\n"
-         "def is_hybrid_model(args): return False\n" + ast.get_source_segment(src, fn), ns)
-    return ns["num_floating_point_operations"]
+
+FLOPS_BASE = dict(num_layers=32, hidden_size=4096, ffn_hidden_size=14336, num_attention_heads=32, num_query_groups=8, kv_channels=128, vocab_size=128256, seq_length=8192)
+_MLA = dict(q_lora_rank=1536, kv_lora_rank=512, qk_head_dim=128, qk_pos_emb_head_dim=64, v_head_dim=128)
+_LIN = dict(linear_key_head_dim=128, linear_value_head_dim=128, linear_num_key_heads=16, linear_num_value_heads=32, linear_conv_kernel_dim=4)
+_THD_LENS = [1000, 3000, 4192] * 2
+# name: (keyword arguments of our model on top of FLOPS_BASE, overrides of the reference's argument namespace, batch size, extra keywords of the reference's call)
+FLOPS_CASES = {
+    "llama3_8b": (dict(batch_size=4), {}, 4, {}),
+    "moe_shared_expert": (dict(seq_length=4096, vocab_size=32000, batch_size=8, num_moe_experts=8, moe_router_topk=2, moe_shared_expert_intermediate_size=2048),
+                          dict(num_experts=8, moe_router_topk=2, seq_length=4096, padded_vocab_size=32000, moe_shared_expert_intermediate_size=2048), 8, {}),
+    "interleaved_moe_mtp": (dict(batch_size=2, num_moe_experts=16, moe_router_topk=4, moe_layer_freq=[0, 1] * 16, moe_ffn_hidden_size=2048, mtp_num_layers=1),
+                            dict(num_experts=16, moe_router_topk=4, moe_layer_freq=[0, 1] * 16, moe_ffn_hidden_size=2048, mtp_num_layers=1), 2, {}),
+    "mla": (dict(num_query_groups=32, batch_size=2, multi_latent_attention=True, **_MLA), dict(multi_latent_attention=True, group_query_attention=False, num_query_groups=32, **_MLA), 2, {}),
+    # THD: real tokens and sum of squared sub-sequence lengths
+    "thd": (dict(batch_size=2, seq_lens=_THD_LENS), {}, 2, dict(seqlen_squared_sum_in_batch=sum(n * n for n in _THD_LENS), total_real_tokens_in_batch=sum(_THD_LENS))),
+    # gated-delta-net linear attention every layer but each 4th
+    "gated_delta_net": (dict(batch_size=2, linear_attention_freq=4), dict(experimental_attention_variant="gated_delta_net", linear_attention_freq=4, **_LIN), 2, {}),
+}
 
 
 def test_flops_model_matches_reference_accounting():
-    import argparse
-
-    import pytest
-
+    """The analytic FLOP count equals the reference's ``num_floating_point_operations`` (values stored in ``tests/golden/reference/training.json``)."""
     from megatron_b200.training.flops import causal_pairs, num_floating_point_operations as ours
 
-    ref = _reference_flops_fn()
-    if ref is None:
-        pytest.skip("reference sources not available")
-
-    def A(**k):
-        d = dict(seq_length=8192, hidden_size=4096, num_layers=32, ffn_hidden_size=14336, num_attention_heads=32, group_query_attention=True, num_query_groups=8, kv_channels=128,
-                 padded_vocab_size=128256, swiglu=True, num_experts=None, moe_layer_freq=1, moe_router_topk=1, moe_ffn_hidden_size=None, moe_latent_size=None,
-                 moe_shared_expert_intermediate_size=None, mtp_num_layers=None, multi_latent_attention=False, experimental_attention_variant=None, attention_output_gate=False,
-                 hybrid_layer_pattern=None)
-        d.update(k)
-        return argparse.Namespace(**d)
-
-    base = dict(num_layers=32, hidden_size=4096, ffn_hidden_size=14336, num_attention_heads=32, num_query_groups=8, kv_channels=128, vocab_size=128256, seq_length=8192)
+    want = _reference_golden("training.json")["flops"]
+    assert sorted(want) == sorted(FLOPS_CASES)
     close = lambda a, b: abs(a - b) <= 1e-9 * abs(b)
-    assert close(ours(**base, batch_size=4), ref(A(), 4))                                                                  # Llama-3 8B
-    assert close(ours(**{**base, "seq_length": 4096, "vocab_size": 32000}, batch_size=8, num_moe_experts=8, moe_router_topk=2, moe_shared_expert_intermediate_size=2048),
-                 ref(A(num_experts=8, moe_router_topk=2, seq_length=4096, padded_vocab_size=32000, moe_shared_expert_intermediate_size=2048), 8))   # MoE + shared expert
-    assert close(ours(**base, batch_size=2, num_moe_experts=16, moe_router_topk=4, moe_layer_freq=[0, 1] * 16, moe_ffn_hidden_size=2048, mtp_num_layers=1),
-                 ref(A(num_experts=16, moe_router_topk=4, moe_layer_freq=[0, 1] * 16, moe_ffn_hidden_size=2048, mtp_num_layers=1), 2))             # interleaved MoE + MTP
-    mla = dict(q_lora_rank=1536, kv_lora_rank=512, qk_head_dim=128, qk_pos_emb_head_dim=64, v_head_dim=128)
-    assert close(ours(**{**base, "num_query_groups": 32}, batch_size=2, multi_latent_attention=True, **mla),
-                 ref(A(multi_latent_attention=True, group_query_attention=False, num_query_groups=32, **mla), 2))                                  # MLA
-    # THD: real tokens and sum of squared sub-sequence lengths
-    lens = [1000, 3000, 4192] * 2
-    assert close(ours(**base, batch_size=2, seq_lens=lens), ref(A(), 2, seqlen_squared_sum_in_batch=sum(l * l for l in lens), total_real_tokens_in_batch=sum(lens)))
-    # gated-delta-net linear attention every layer but each 4th
-    lin = dict(linear_key_head_dim=128, linear_value_head_dim=128, linear_num_key_heads=16, linear_num_value_heads=32, linear_conv_kernel_dim=4)
-    assert close(ours(**base, batch_size=2, linear_attention_freq=4),
-                 ref(A(experimental_attention_variant="gated_delta_net", linear_attention_freq=4, **lin), 2))
+    for name, (kw, _, _, _) in FLOPS_CASES.items():
+        assert close(ours(**{**FLOPS_BASE, **kw}), want[name]), name
+    base = FLOPS_BASE
     # sliding window (ours only): never more than full causal attention, equal when the window covers the sequence
     assert ours(**base, batch_size=1, window_size=(1024, 0)) < ours(**base, batch_size=1) == ours(**base, batch_size=1, window_size=(8192, 0))
     assert causal_pairs(10, 4) == 4 * 10 - 8
@@ -603,18 +585,9 @@ def test_tokenizer_flags_and_vocab_padding():
 
 
 def test_every_flag_of_the_reference_runtime_parser_is_accepted():
-    """Build the reference's REAL parser (dataclass-generated groups included) in a subprocess and check each option string parses here with the same arity."""
-    import json
-    import subprocess
-    import sys
-
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    if not os.path.isdir(os.path.join(root, "baseline", "_ref", "megatron")) or not os.path.isdir("/root/reference/megatron/training"):
-        pytest.skip("reference not installed")
-    sys.path.insert(0, os.path.join(root, "tools"))
-    from gen_reference_flag_table import _introspect
-
-    ref = _introspect("/root/reference")
+    """Each option string of the reference's REAL parser (dataclass-generated groups included; stored in ``tests/golden/reference/training.json``) parses here
+    with the same arity."""
+    ref = [{"flags": flags, "nargs": nargs} for flags, nargs in _reference_golden("training.json")["parser_flags"]]
     assert len(ref) > 700
     from megatron_b200.training.arguments import build_full_parser
 

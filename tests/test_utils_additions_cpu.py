@@ -125,9 +125,14 @@ def test_transformer_utils_additions():
     assert cfg.cuda_graph_impl == "full"
 
 
+# a small fixed checkpoint directory whose integrity manifest the unmodified reference wrote into tests/golden/reference/integrity.json
+INTEGRITY_FILES = {"__0_0.distcp": bytes(range(256)) * 5, "common.pt": b"common state", "metadata.json": b'{"sharded_backend": "torch_dist"}'}
+
+
 def test_checkpoint_integrity_manifest_and_strict_helpers(tmp_path):
+    import json
     import os
-    import sys
+    import shutil
 
     from megatron_b200.core import dist_checkpointing as dc
     from megatron_b200.core.dist_checkpointing import validation as V
@@ -143,14 +148,17 @@ def test_checkpoint_integrity_manifest_and_strict_helpers(tmp_path):
         V.verify_checkpoint(str(tmp_path / "nope"))
     V.save_integrity_manifest(ck)
     V.verify_integrity_manifest(ck)
-    ref = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "baseline", "_ref")
-    if os.path.isdir(ref):                                   # the unmodified reference accepts our manifest
-        sys.path.insert(0, ref)
-        try:
-            from megatron.core.dist_checkpointing.validation import verify_integrity_manifest as ref_verify
-            ref_verify(ck)
-        finally:
-            sys.path.remove(ref)
+    # the unmodified reference writes the same manifest for the same files (tests/golden/reference/integrity.json), and ours accepts the reference's
+    fixed = tmp_path / "fixed"
+    fixed.mkdir()
+    for name, data in INTEGRITY_FILES.items():
+        (fixed / name).write_bytes(data)
+    V.save_integrity_manifest(str(fixed))
+    golden = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference", "integrity.json")
+    with open(golden) as f, open(fixed / "integrity.json") as g:
+        assert json.load(g) == json.load(f)
+    shutil.copyfile(golden, fixed / "integrity.json")
+    V.verify_integrity_manifest(str(fixed))
     victim = next(n for n in sorted(os.listdir(ck)) if n.endswith(".distcp"))
     with open(os.path.join(ck, victim), "r+b") as f:
         f.seek(10)
